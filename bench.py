@@ -46,7 +46,42 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true",
                     help="skip the other target configurations (synthetic-3m; at N > 1 also the index-sharded run) that the default "
                          "eurlex-4k run reports under `secondary`")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload returned as DIR/<name>.npy (rank 0), so that two "
+                         "builds can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Saves `arrays` ({name: float32 or float64 array}) as out_dir/<name>.npy; refuses to write more than DUMP_LIMIT_BYTES."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def csr_result_arrays(Y, max_bytes=DUMP_LIMIT_BYTES, seed=0):
+    """The CSR result of an XR-Linear prediction as float arrays (row pointers and label ids exactly representable in float64).
+    A result larger than `max_bytes` is cut to a fixed, seeded sample of its rows (row ids saved beside it)."""
+    import scipy.sparse as smat
+
+    Y = smat.csr_matrix(Y)
+    rows = np.arange(Y.shape[0])
+    per_row = 12.0 * Y.nnz / max(Y.shape[0], 1) + 16.0
+    if per_row * Y.shape[0] > max_bytes:
+        rows = np.sort(np.random.default_rng(seed).choice(Y.shape[0], size=int(max_bytes // per_row), replace=False))
+        Y = Y[rows]
+    return {"rows": rows.astype(np.float64), "indptr": Y.indptr.astype(np.float64), "labels": Y.indices.astype(np.float64),
+            "scores": Y.data.astype(np.float32)}
 
 
 def dist_env():
@@ -518,7 +553,7 @@ def hnsw_time_reference(folder, Q, cfg, steps, warmup, budget_s=60.0):
             "sample": f"{sample.shape[0]} of {Q.shape[0]} queries per step, {steps} steps, {n_cores} searchers (all host threads)"}
 
 
-def measure_hnsw(args, workload, rank, n_gpus, local, dist, barrier, steps, warmup, with_cpu=True):
+def measure_hnsw(args, workload, rank, n_gpus, local, dist, barrier, steps, warmup, with_cpu=True, dump_dir=None):
     """One HNSW workload on this rank's GPU (replicas: every rank its own query batch, same index file); returns the JSON line as
     a dict on rank 0 (None elsewhere)."""
     from ctypes import POINTER, byref, c_float, c_uint32, c_uint64
@@ -609,6 +644,8 @@ def measure_hnsw(args, workload, rank, n_gpus, local, dist, barrier, steps, warm
     gi = np.zeros((nq, topk), dtype=np.uint32)
     gd = np.zeros((nq, topk), dtype=np.float32)
     c.pb200_hnsw_resident_fetch(h, gi.ctypes.data_as(POINTER(c_uint32)), gd.ctypes.data_as(POINTER(c_float)))
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"neighbours": gi.astype(np.float64), "distances": gd})
     parity = {"checked_queries": 0, "checker": "unavailable (oracle/_ref absent)"}
     import oracle
 
@@ -762,7 +799,7 @@ def main_hnsw(args):
             dist.barrier()
 
     barrier()
-    line = measure_hnsw(args, args.workload, rank, n_gpus, local, dist, barrier, args.steps, args.warmup)
+    line = measure_hnsw(args, args.workload, rank, n_gpus, local, dist, barrier, args.steps, args.warmup, dump_dir=args.dump_outputs)
     if rank == 0:
         print(json.dumps(line))
     if dist is not None:
@@ -826,7 +863,7 @@ def _ncu_notes(workload, kernel):
 
 
 def measure_xlinear(args, workload, rank, n_gpus, local, dist, barrier, lib, steps, warmup, strong=False, with_cpu=True,
-                    with_clocks=True):
+                    with_clocks=True, dump_dir=None):
     """One XR-Linear workload on this rank's GPU.  strong=False: every rank its own batch of the workload's shape (weak
     scaling, replicas); strong=True: ONE batch of the workload's size, rows split over the ranks by nnz (strong scaling).
     Returns the JSON-able record (rank 0) -- parity-gated: raises if the GPU result differs from the reference."""
@@ -895,6 +932,8 @@ def measure_xlinear(args, workload, rank, n_gpus, local, dist, barrier, lib, ste
     c.pb200_xlinear_resident_fetch(h, fetch.cfunc)
     got_resident = fetch.get()
     parity = parity_gate_xlinear(got_resident, folder, X, cfg, rows=(1024 if rank == 0 else 128), what=f"{workload} resident batch")
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, csr_result_arrays(got_resident))
 
     # ------------------------------------------------------------ per-kernel timing (CUDA events on the launch stream)
     c.pb200_xlinear_set_profile(h, 1)
@@ -1096,7 +1135,8 @@ def main():
     lib.require_gpu()
     lib.set_device(local)
 
-    line, keep = measure_xlinear(args, args.workload, rank, n_gpus, local, dist, barrier, lib, args.steps, args.warmup)
+    line, keep = measure_xlinear(args, args.workload, rank, n_gpus, local, dist, barrier, lib, args.steps, args.warmup,
+                                 dump_dir=args.dump_outputs)
     del keep
 
     # ------------------------------------------------------------ the other target configurations, in the same run

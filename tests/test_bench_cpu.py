@@ -91,3 +91,37 @@ def test_sparse_row_generator_is_deterministic_and_canonical():
     assert (A != B).nnz == 0 and A.has_canonical_format and A.dtype == np.float32
     assert 30 < A.nnz / A.shape[0] < 45
     assert np.allclose(np.sqrt(np.asarray(A.multiply(A).sum(axis=1)).ravel()), 1.0, atol=1e-5)
+
+
+def test_dump_outputs_writes_float_arrays_within_the_limit(tmp_path):
+    """--dump-outputs: the csr result of the timed step round-trips through float arrays; a result over the byte limit is cut to
+    the same seeded sample of rows every time; nothing over the limit is written."""
+    import importlib.util
+
+    import scipy.sparse as smat
+
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    argv, sys.argv = sys.argv, ["bench.py"]
+    try:
+        spec.loader.exec_module(b)
+    finally:
+        sys.argv = argv
+    Y = smat.random(300, 5000, density=0.002, format="csr", dtype=np.float32, random_state=3)
+    full = b.csr_result_arrays(Y)
+    b.dump_outputs(str(tmp_path / "full"), full)
+    got = {k: np.load(str(tmp_path / "full" / (k + ".npy"))) for k in full}
+    assert all(got[k].dtype in (np.float32, np.float64) for k in got)
+    back = smat.csr_matrix((got["scores"], got["labels"].astype(np.int64), got["indptr"].astype(np.int64)), shape=Y.shape)
+    assert (back != Y).nnz == 0 and np.array_equal(got["rows"], np.arange(300))
+    small, again = b.csr_result_arrays(Y, max_bytes=4096), b.csr_result_arrays(Y, max_bytes=4096)
+    assert 0 < small["rows"].size < 300 and sum(a.nbytes for a in small.values()) <= 4096
+    assert all(np.array_equal(small[k], again[k]) for k in small)
+    rows = small["rows"].astype(np.int64)
+    assert (smat.csr_matrix((small["scores"], small["labels"].astype(np.int64), small["indptr"].astype(np.int64)),
+                            shape=(rows.size, Y.shape[1])) != Y[rows]).nnz == 0
+    with pytest.raises(RuntimeError):
+        b.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(b.DUMP_LIMIT_BYTES // 8 + 1)})
+    assert not os.path.exists(str(tmp_path / "big"))
+    r = _run(["--steps", "0"])
+    assert r.returncode != 0 and "--steps" in r.stderr

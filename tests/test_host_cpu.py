@@ -196,9 +196,12 @@ def test_single_layer_model_from_in_memory_csc_equals_the_folder_loader(clib, tm
 @pytest.mark.parametrize("permute,prune,bias", [(False, 0.0, 1.0), (True, 0.25, 1.0), (False, 0.0, -1.0)])
 def test_mmap_writer_output_loads_in_the_reference_library(tmp_path, clib, have_ref, permute, prune, bias):
     """c_xlinear_compile_mmap_model of THIS library (host-only writer, pecos_b200/csrc/xlinear_host.h write_xlinear_mmap_model):
-    the folder it writes must load in the REFERENCE library and predict exactly what the reference predicts from the npz model
-    (and from its own compiled copy); our own mmap loader must read it back to the same chunked layout."""
-    from .util import assert_csr_parity, random_tree
+    our own mmap loader must read the folder it writes back to the same chunked layout as the npz model and as the folder the
+    REFERENCE's own writer makes from it (recorded under tests/golden/ref_results/), and -- where oracle/_ref is built -- the
+    reference library must load it and predict exactly what it predicts from the npz model."""
+    from .util import RecordedReference, assert_csr_parity, random_tree
+
+    rec = RecordedReference(f"mmap_writer_{int(permute)}_{prune}_{bias}")
 
     folder = str(tmp_path / "m")
     layers = random_tree(77, [5, 30, 400], 300, 20, bias=bias, permute=permute, prune=prune)
@@ -211,18 +214,22 @@ def test_mmap_writer_output_loads_in_the_reference_library(tmp_path, clib, have_
     for la, lb in zip(a, b):
         for key in la:
             assert np.array_equal(np.asarray(la[key]), np.asarray(lb[key])), key
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
     from oracle import ref
 
-    X = synth.make_queries(78, 60, 300, 25)
-    want = ref.RefXLinear(os.path.join(folder, "ranker")).predict(X, 6, None, 5)
-    got = ref.RefXLinear(os.path.join(ours, "ranker"), is_mmap=True).predict(X, 6, None, 5)
-    assert_csr_parity(got, want, rtol=0.0, what="reference library on the folder written by pecos_b200")
-    theirs = str(tmp_path / "theirs")
-    os.makedirs(theirs)
-    ref.compile_mmap_model(os.path.join(folder, "ranker"), os.path.join(theirs, "ranker"))
+    if have_ref:
+        X = synth.make_queries(78, 60, 300, 25)
+        want = ref.RefXLinear(os.path.join(folder, "ranker")).predict(X, 6, None, 5)
+        got = ref.RefXLinear(os.path.join(ours, "ranker"), is_mmap=True).predict(X, 6, None, 5)
+        assert_csr_parity(got, want, rtol=0.0, what="reference library on the folder written by pecos_b200")
+
+    def write(path):
+        os.makedirs(path)
+        ref.compile_mmap_model(os.path.join(folder, "ranker"), os.path.join(path, "ranker"))
+
+    theirs = rec.folder("theirs", write)
+    rec.save()
     c = clib.host_model_layout(os.path.join(theirs, "ranker"), is_mmap=True)
+    assert len(c) == len(b)
     for lb, lc in zip(b, c):
         for key in lb:
             assert np.array_equal(np.asarray(lb[key]), np.asarray(lc[key])), key
@@ -255,13 +262,14 @@ def test_hnsw_host_ingest_of_dense_and_sparse_indices(clib):
 @pytest.mark.parametrize("permute,prune", [(False, 0.0), (True, 0.25)])
 def test_mlmodel_mmap_writer_is_interchangeable_with_the_reference(tmp_path, clib, have_ref, permute, prune):
     """c_mlmodel_compile_mmap_model of THIS library (host-only; pecos_b200/csrc/xlinear_host.h compile_mlmodel_mmap): every layer
-    folder it writes holds the same blocks (W.mmap_store, C.mmap_store) as the reference's output, loads in the reference library and
-    predicts what the reference predicts from its own copy -- incl. the root layer, whose C.npz may be absent."""
-    from .util import assert_csr_parity, random_tree
+    folder it writes holds the same blocks (W.mmap_store, C.mmap_store) as the reference's output (recorded under
+    tests/golden/ref_results/) and -- where oracle/_ref is built -- loads in the reference library and predicts what the reference
+    predicts from its own copy; incl. the root layer, whose C.npz may be absent."""
+    from oracle import ref, restatement
 
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref
+    from .util import RecordedReference, assert_csr_parity, random_tree
+
+    rec = RecordedReference(f"mlmodel_writer_{int(permute)}_{prune}")
 
     folder = str(tmp_path / "m")
     layers = random_tree(91, [4, 24, 300], 200, 18, bias=1.0, permute=permute, prune=prune)
@@ -271,15 +279,16 @@ def test_mlmodel_mmap_writer_is_interchangeable_with_the_reference(tmp_path, cli
         src = os.path.join(folder, "ranker", f"{d}.model")
         if d == 0 and os.path.exists(os.path.join(src, "C.npz")):
             os.remove(os.path.join(src, "C.npz"))  # the root layer's C is optional (inference.hpp:1580-1583)
-        ours, theirs = str(tmp_path / f"ours{d}"), str(tmp_path / f"theirs{d}")
+        ours = str(tmp_path / f"ours{d}")
         ref.compile_mlmodel_mmap(src, ours, clib=clib.clib_float32)
-        ref.compile_mlmodel_mmap(src, theirs)
-        from oracle import restatement
-
+        theirs = rec.folder(f"layer{d}", lambda path: ref.compile_mlmodel_mmap(src, path))
         for f in ("W.mmap_store", "C.mmap_store"):  # block by block (the padding between blocks is not initialised by the reference)
             ba, bb = restatement.read_mmap_store(os.path.join(ours, f)), restatement.read_mmap_store(os.path.join(theirs, f))
             assert len(ba) == len(bb) == 6 and all(np.array_equal(x, y) for x, y in zip(ba, bb)), (d, f)
+        if not have_ref:
+            continue
         a, b = ref.MLModelHandle(ours), ref.MLModelHandle(theirs)
         assert [a.attr(k) for k in ("nr_labels", "nr_codes", "nr_features")] == [b.attr(k) for k in ("nr_labels", "nr_codes", "nr_features")]
         assert_csr_parity(a.predict(X, None, None, 0), b.predict(X, None, None, 0), rtol=0.0, what=f"layer {d}: reference on our folder")
         assert_csr_parity(a.predict(X, None, "sigmoid", 3), b.predict(X, None, "sigmoid", 3), rtol=0.0, what=f"layer {d}: overrides")
+    rec.save()

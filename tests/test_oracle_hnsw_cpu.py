@@ -73,14 +73,19 @@ def test_sparse_hnsw_restatement_reproduces_reference_goldens(built):
     assert n >= 20 and {it["model"] for it in index} >= {"fixture_ip", "ip_tfidf", "l2_tfidf", "ip_short"}
 
 
-def test_sparse_hnsw_restatement_equals_the_reference_library_on_random_indices(built, have_ref, tmp_path):
-    """Live diff against oracle/_ref on freshly trained sparse indices (both metrics), incl. recall of the reference's own test
-    (test/pecos/ann/test_hnsw.py:86-124: recall vs brute force >= 0.99 on the prebuilt sparse fixture)."""
-    if not have_ref:
-        pytest.skip("oracle/_ref not built")
+def test_sparse_hnsw_restatement_equals_the_reference_library_on_random_indices(built):
+    """Diff against oracle/_ref on sparse indices it trained from seeded random rows (both metrics; indices and search results
+    recorded under tests/golden/ref_results/), incl. recall of the reference's own test (test/pecos/ann/test_hnsw.py:86-124: recall
+    vs brute force >= 0.99 on the prebuilt sparse fixture)."""
     import scipy.sparse as smat
 
     from oracle import ref, restatement
+
+    from .util import RecordedReference
+
+    rec = RecordedReference("hnsw_sparse_random")
+    # the restatement follows the distance kernels of the host the reference ran on
+    isa = int(rec.arrays("isa", lambda: (np.int64(restatement.host_isa()),))[0])
 
     sys_path_golden = os.path.join(HERE, "golden")
     import importlib.util
@@ -91,15 +96,18 @@ def test_sparse_hnsw_restatement_equals_the_reference_library_on_random_indices(
     for metric, (N, D, nnz) in (("ip", (1200, 3000, 30)), ("l2", (900, 200, 12))):
         X = mgs.make_rows(7, N, D, nnz, 50)
         Q = mgs.make_rows(8, 40, D, nnz, 9)
-        r = ref.RefHNSW.train(X, M=8, efC=40, metric=metric, threads=1)
-        folder = str(tmp_path / metric)
-        r.save(os.path.join(folder, "c_model"))
-        json.dump({"data_type": "csr", "metric_type": metric}, open(os.path.join(folder, "param.json"), "w"))
-        o = restatement.OracleHNSW(folder, isa=restatement.host_isa())
+        r = ref.RefHNSW.train(X, M=8, efC=40, metric=metric, threads=1) if rec.recording else None
+
+        def write(folder):
+            r.save(os.path.join(folder, "c_model"))
+            json.dump({"data_type": "csr", "metric_type": metric}, open(os.path.join(folder, "param.json"), "w"))
+
+        o = restatement.OracleHNSW(rec.folder(metric, write), isa=isa)
         assert abs(o.vectors() - X).max() == 0
         for efS, topk in ((30, 10), (120, 20)):
-            a, b = o.predict(Q, efS, topk), r.predict(Q, efS, topk)
+            a, b = o.predict(Q, efS, topk), rec.arrays(f"{metric} {efS} {topk}", lambda: r.predict(Q, efS, topk))
             assert np.array_equal(a[0], b[0]) and np.array_equal(a[1].view(np.uint32), b[1].view(np.uint32))
+    rec.save()
     # recall on the reference's fixture
     fx = os.path.join(SPARSE, "fixture_ip")
     o = restatement.OracleHNSW(fx, isa=0)

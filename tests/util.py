@@ -1,10 +1,63 @@
 """Shared helpers for the parity tests (test infrastructure)."""
 import os
+import shutil
 
 import numpy as np
 import scipy.sparse as smat
 
 from pecos_b200 import synth
+
+REF_RESULTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_results")
+
+
+class RecordedReference(object):
+    """What the reference library (oracle/_ref) returned for one test's seeded inputs, stored under tests/golden/ref_results/<name>
+    so that the test compares with the reference without needing it at test time.
+
+    With PB200_RECORD_REFERENCE=1 (and oracle/_ref built) every call runs the reference, stores its result and returns it; `save()`
+    then writes the recording.  Otherwise the stored result is returned and the reference is never called."""
+
+    def __init__(self, name):
+        self.dir = os.path.join(REF_RESULTS, name)
+        self.recording = os.environ.get("PB200_RECORD_REFERENCE") == "1"
+        self.store = {}
+        if self.recording:
+            shutil.rmtree(self.dir, ignore_errors=True)
+            os.makedirs(self.dir)
+        else:
+            with np.load(os.path.join(self.dir, "results.npz")) as f:
+                self.store = dict(f)
+
+    def csr(self, key, compute):
+        """A csr result (ids, stored order and score bits are kept)."""
+        if self.recording:
+            Y = smat.csr_matrix(compute())
+            self.store.update({key + "|indptr": Y.indptr.astype(np.int32), key + "|indices": Y.indices.astype(np.int32),
+                               key + "|data": Y.data.astype(np.float32), key + "|shape": np.asarray(Y.shape, dtype=np.int64)})
+            return Y
+        s = self.store
+        return smat.csr_matrix((s[key + "|data"], s[key + "|indices"], s[key + "|indptr"]), shape=tuple(s[key + "|shape"]))
+
+    def arrays(self, key, compute):
+        """A tuple of dense arrays, returned with the dtypes they were recorded with."""
+        if self.recording:
+            out = tuple(np.asarray(a) for a in compute())
+            self.store.update({f"{key}|{i}": a for i, a in enumerate(out)})
+            return out
+        n = sum(1 for k in self.store if k.startswith(key + "|"))
+        return tuple(self.store[f"{key}|{i}"] for i in range(n))
+
+    def folder(self, key, write):
+        """A folder the reference writes (an index, a compiled model): `write(path)` when recording, the stored copy otherwise."""
+        path = os.path.join(self.dir, key)
+        if self.recording:
+            write(path)
+        assert os.path.isdir(path), path
+        return path
+
+    def save(self):
+        if self.recording:
+            np.savez_compressed(os.path.join(self.dir, "results.npz"), **self.store)
 
 
 def assert_csr_parity(got, want, rtol=1e-5, what=""):
