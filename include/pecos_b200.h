@@ -293,6 +293,23 @@ void pb200_hnsw_get_info(void* model_ptr, uint64_t* out);
  * strictly ascending in-range indices).  metric 0 = ip, 1 = l2; sparse 0 = drm, 1 = csr.  Returns 0 and
  * out[8] = {num_node, feat_dim, maxM, maxM0, max_level, init_node, stored vector entries, level-0 degree sum}, or 1 (reason on stderr). */
 int pb200_hnsw_host_info(const char* model_dir, int metric, int sparse, uint64_t* out);
+/* Distance work of the GPU builder for SPARSE (csr) indices (pecos_b200/hnsw_build.py).  All pointers are CALLER-OWNED DEVICE
+ * buffers; the kernels are enqueued on `stream` (a cudaStream_t, e.g. torch.cuda.current_stream().cuda_stream) of `device` and
+ * the calls return without synchronising.  Distances have the reference's bits (FeatVecSparse{IP,L2}Simd::distance: ordered
+ * sum of the matched products; ip = 1 - dot, l2 = -2 dot); orders are by (distance, id).  metric 0 = ip, 1 = l2.  Rows are a
+ * canonical csr (row_ptr i64 [n+1], col_idx i32 ascending per row, val f32).  Both return 0, or 1 (reason on stderr).
+ *   knn:    for every row q < n, its k nearest rows among 0..q-1.  post_ptr i64 [cols+1] / post_entries {i32 row, f32 value}
+ *           [nnz] are the posting lists (csc, rows ascending), self_pos i64 [nnz] the position of every csr entry in its
+ *           posting list, cursor i64 [nnz] scratch.  out_keys i64 [n][k] ascending: (orderable(distance) << 32 | row) with
+ *           the sign bit flipped (signed order = key order); INT64_MAX pads rows with fewer than k earlier rows.
+ *   select: the neighbour-selection heuristic (hnsw.hpp:556-592) for n nodes: cand i64 [n][C] global row ids (-1 = empty),
+ *           ascending by (cand_d f32 [n][C], id); keep u8 [n][C] receives 1 for the kept candidates (at most cap). */
+int pb200_hnsw_build_sparse_knn(int device, void* stream, uint32_t n, uint32_t k, int metric, const void* row_ptr,
+                                const void* col_idx, const void* val, const void* post_ptr, const void* post_entries,
+                                const void* self_pos, void* cursor, void* out_keys);
+int pb200_hnsw_build_sparse_select(int device, void* stream, uint32_t n, uint32_t C, uint32_t cap, int metric,
+                                   const void* row_ptr, const void* col_idx, const void* val, const void* cand,
+                                   const void* cand_d, void* keep);
 /* A query whose candidate queue outgrows the per-warp scratch (PB200_HNSW_VCAP entries, default 32768) makes the engine re-run
  * the batch with twice the capacity (up to num_node + 1, which cannot overflow) -- this counts those re-runs. */
 uint32_t pb200_hnsw_vcap_retries(void* model_ptr);

@@ -474,6 +474,8 @@ class B200CoreLib(object):
         fp(c.pb200_hnsw_set_stages, c_int, [c_void_p, c_int])
         fp(c.pb200_hnsw_get_info, None, [c_void_p, POINTER(c_uint64)])
         fp(c.pb200_hnsw_host_info, c_int, [c_char_p, c_int, c_int, POINTER(c_uint64)])
+        fp(c.pb200_hnsw_build_sparse_knn, c_int, [c_int, c_void_p, c_uint32, c_uint32, c_int] + [c_void_p] * 8)
+        fp(c.pb200_hnsw_build_sparse_select, c_int, [c_int, c_void_p, c_uint32, c_uint32, c_uint32, c_int] + [c_void_p] * 6)
         fp(c.pb200_xlinear_host_load, c_void_p, [c_char_p, c_int])
         fp(c.pb200_xlinear_host_free, None, [c_void_p])
         fp(c.pb200_xlinear_host_depth, c_uint32, [c_void_p])

@@ -12,8 +12,9 @@ ret_csr=True)``                                ``(indices, distances)`` arrays
 ``HNSW.searchers_create(n)`` / ``Searchers``   opaque scratch token (the per-warp scratch lives with the engine)
 =============================================  =======================================================
 
-Index construction stays on the reference CPU library (dense indices can also be built on the GPU:
-``pecos_b200.hnsw_build``).  Served index kinds: dense ``drm`` and sparse ``csr`` float32 with the ``ip`` or ``l2`` metric
+Index construction stays on the reference CPU library; both index kinds can also be built on the GPU by
+``pecos_b200.hnsw_build.build_hnsw_index`` (dense rows: tiled GEMMs; ``scipy.sparse`` rows: the exact sparse kernels of
+``csrc/hnsw_build_sparse.cu``), which writes files that this class and the reference both load.  Served index kinds: dense ``drm`` and sparse ``csr`` float32 with the ``ip`` or ``l2`` metric
 (csr rows: column indices strictly ascending -- queries are canonicalised with ``sum_duplicates()`` / ``sort_indices()``
 when needed).  There is no CPU fallback: loading without a visible CUDA device raises ``RuntimeError``.
 """

@@ -27,6 +27,10 @@ instead of 10^9 dependent single-vector distance calls):
 5. neighbour lists sorted by ascending distance (hnsw.hpp:823-845), records laid out as GraphL0 / GraphL1 store them.
 
 torch is used for device memory and the GEMM / top-k primitives; nothing here is on the search path.
+
+A ``scipy.sparse`` input builds a sparse (csr) index with the same steps, on the GPU only (``_build_sparse``): the distance work
+is the CUDA kernels of ``csrc/hnsw_build_sparse.cu`` (exact prefix kNN as an SpGEMM over posting lists, the heuristic one warp
+per node), every distance in the reference's exact bits, every order by (distance, id) -- the build is deterministic.
 """
 import json
 import math
@@ -150,16 +154,16 @@ def _heuristic(torch, X, node_pos, cand, cand_d, cap, metric, tile):
     return kept_all
 
 
-def _build_level(torch, X, ids, M, cap, efC, metric, q_tile, c_tile, h_tile):
-    """Neighbour lists (global ids, ascending distance, <= cap each) of the nodes `ids` on one level."""
+def _link_level(torch, ids, pos, dist, M, cap, heuristic):
+    """The distance-independent half of a level: forward selection, reverse links, pruning of over-full pools and
+    compaction.  pos / dist [n, k]: every node's kNN among the earlier nodes of `ids` (positions into `ids`, ascending by
+    (distance, id); -1 / inf = empty); heuristic(cand [m, C] global ids, cand_d [m, C], cap) -> kept mask [m, C].
+    Returns the neighbour lists [n, cap] (global ids, ascending distance, -1 = empty) and the degrees."""
     n = ids.numel()
-    dev = X.device
+    dev = ids.device
     lists = torch.full((n, cap), -1, dtype=torch.long, device=dev)
-    if n <= 1:
-        return lists, torch.zeros(n, dtype=torch.long, device=dev)
-    pos, dist = _exact_knn(torch, X, ids, efC, metric, q_tile, c_tile)          # positions into ids
     cand = torch.where(pos >= 0, ids[pos.clamp_min(0)], torch.full_like(pos, -1))
-    keep = _heuristic(torch, X, ids, cand, dist, M, metric, h_tile)            # forward selection: at most M (hnsw.hpp:598)
+    keep = heuristic(cand, dist, M)                                            # forward selection: at most M (hnsw.hpp:598)
     # edges u -> v (selected) and the offers v <- u
     src = torch.arange(n, device=dev).unsqueeze(1).expand_as(cand)[keep]       # positions
     dst_pos = pos[keep]
@@ -192,7 +196,7 @@ def _build_level(torch, X, ids, M, cap, efC, metric, q_tile, c_tile, h_tile):
     keep2 = pool >= 0
     if bool(over.any()):
         idx = torch.nonzero(over).squeeze(1)
-        keep2[idx] = _heuristic(torch, X, ids[idx], pool[idx], pool_d[idx], cap, metric, h_tile)
+        keep2[idx] = heuristic(pool[idx], pool_d[idx], cap)
     # compact the kept neighbours (already ascending by distance)
     rank2 = torch.cumsum(keep2.long(), 1) - 1
     rows = torch.arange(n, device=dev).unsqueeze(1).expand_as(pool)
@@ -201,16 +205,32 @@ def _build_level(torch, X, ids, M, cap, efC, metric, q_tile, c_tile, h_tile):
     return lists, sel.sum(1)
 
 
+def _build_level(torch, X, ids, M, cap, efC, metric, q_tile, c_tile, h_tile):
+    """Neighbour lists (global ids, ascending distance, <= cap each) of the nodes `ids` on one level."""
+    n = ids.numel()
+    dev = X.device
+    if n <= 1:
+        return torch.full((n, cap), -1, dtype=torch.long, device=dev), torch.zeros(n, dtype=torch.long, device=dev)
+    pos, dist = _exact_knn(torch, X, ids, efC, metric, q_tile, c_tile)          # positions into ids
+    return _link_level(torch, ids, pos, dist, M, cap,
+                       lambda cand, cand_d, m: _heuristic(torch, X, None, cand, cand_d, m, metric, h_tile))
+
+
 # ------------------------------------------------------------------------------------------------ public entry point
 def build_hnsw_index(X, folder, M=32, efC=100, metric="ip", seed=0, max_level_upper_bound=-1, device=None, pred_kwargs=None,
                      q_tile=4096, c_tile=65536, h_tile=None, allow_tf32=False):
-    """Builds the index for the rows of ``X`` (float32 [N, d]) and writes it to ``folder`` in the reference's format.
-    Returns a dict with the build statistics.  ``device``: torch device (default: cuda:0; "cpu" is accepted for tiny inputs,
-    e.g. format tests on a box without a GPU)."""
+    """Builds the index for the rows of ``X`` and writes it to ``folder`` in the reference's format.  Returns a dict with the
+    build statistics.
+
+    ``X``: float32 [N, d] (dense ``drm`` index), or a ``scipy.sparse`` matrix (sparse ``csr`` index, built by the CUDA kernels
+    of ``csrc/hnsw_build_sparse.cu``; see ``_build_sparse``).  ``device``: torch device (default: cuda:0).  For dense ``X``,
+    "cpu" is accepted for tiny inputs, e.g. format tests on a box without a GPU; a sparse ``X`` needs a GPU."""
     import torch
 
     if metric not in _HNSW_T:
         raise ValueError(f"metric must be 'ip' or 'l2', got {metric!r}")
+    if _is_sparse(X):
+        return _build_sparse(X, folder, M, efC, metric, seed, max_level_upper_bound, device, pred_kwargs)
     X = np.ascontiguousarray(X, dtype=np.float32)
     N, d = X.shape
     if N < 1:
@@ -223,13 +243,7 @@ def build_hnsw_index(X, folder, M=32, efC=100, metric="ip", seed=0, max_level_up
         h_tile = max(16, min(2048, (256 << 20) // (4 * max(4 * maxM0, 64) * max(4 * maxM0, 64, d))))
 
     # 1. levels (hnsw.hpp:785-793) and the entry point
-    rng = np.random.default_rng(seed)
-    u = 1.0 - rng.random(N)  # (0, 1]
-    levels = np.floor(-np.log(u) * (1.0 / math.log(float(maxM)))).astype(np.int64)
-    if max_level_upper_bound >= 0:
-        levels = np.minimum(levels, int(max_level_upper_bound))
-    max_level = int(levels.max())
-    init_node = int(np.argmax(levels == max_level))
+    levels, max_level, init_node = _levels(N, maxM, seed, max_level_upper_bound)
 
     Xd = torch.from_numpy(X).to(dev)
     lvl = torch.from_numpy(levels).to(dev)
@@ -252,7 +266,32 @@ def build_hnsw_index(X, folder, M=32, efC=100, metric="ip", seed=0, max_level_up
     l0[:, 4 * (1 + maxM0): 4 * (1 + maxM0) + 4] = np.full((N, 1), d, dtype="<u4").view(np.uint8)
     l0[:, 4 * (1 + maxM0) + 4:] = X.view(np.uint8).reshape(N, 4 * d)
     mem_start = (np.arange(N + 1, dtype="<u8") * rec)
-    # GraphL1: per node max_level slots of [deg u32][maxM ids u32] (hnsw.hpp:188-219); every node gets all slots
+    node_mem, level_mem, l1 = _graph_l1(N, max_level, maxM, level_lists)
+
+    # 3. files
+    blocks = [_scalar(N), _scalar(maxM), _scalar(maxM0), _scalar(int(efC)), _scalar(max_level), _scalar(init_node),
+              _scalar(N), _scalar(d), _scalar(maxM0), _scalar(rec)] + _vector(mem_start) + _vector(l0.reshape(-1)) + \
+             [_scalar(N), _scalar(max_level), _scalar(maxM), _scalar(node_mem), _scalar(level_mem)] + _vector(l1)
+    _write_folder(folder, blocks, _HNSW_T[metric], "drm", metric, N, d, maxM, maxM0, int(efC), max_level, init_node, pred_kwargs,
+                  "pecos_b200.hnsw_build (batch, exact kNN + heuristic)")
+    return {"num_node": N, "feat_dim": d, "max_level": max_level, "init_node": init_node,
+            "mean_degree_l0": float(deg0.mean()), "nodes_per_level": [int(t[0].size) for t in level_lists]}
+
+
+def _levels(N, maxM, seed, max_level_upper_bound):
+    """Node levels as the reference draws them (hnsw.hpp:785-793) and the entry point (first node of the top level)."""
+    rng = np.random.default_rng(seed)
+    u = 1.0 - rng.random(N)  # (0, 1]
+    levels = np.floor(-np.log(u) * (1.0 / math.log(float(maxM)))).astype(np.int64)
+    if max_level_upper_bound >= 0:
+        levels = np.minimum(levels, int(max_level_upper_bound))
+    max_level = int(levels.max())
+    return levels, max_level, int(np.argmax(levels == max_level))
+
+
+def _graph_l1(N, max_level, maxM, level_lists):
+    """GraphL1: per node max_level slots of [deg u32][maxM ids u32] (hnsw.hpp:188-219); every node gets all slots, slots
+    beyond a node's degree are zero.  level_lists[l] = (ids, lists [n, >= maxM] global ids / -1, degrees)."""
     level_mem = 1 + maxM
     node_mem = max_level * level_mem
     l1 = np.zeros(N * node_mem, dtype="<u4")
@@ -262,23 +301,270 @@ def build_hnsw_index(X, folder, M=32, efC=100, metric="ip", seed=0, max_level_up
         l1[base] = deg_l
         cols = np.where(lists_l >= 0, lists_l, 0).astype("<u4")
         l1[(base[:, None] + 1 + np.arange(maxM)[None, :]).ravel()] = cols.ravel()
+    return node_mem, level_mem, l1
 
-    # 3. files
+
+def _write_folder(folder, blocks, hnsw_t, data_type, metric, N, d, maxM, maxM0, efC, max_level, init_node, pred_kwargs, builder):
     c_model = os.path.join(folder, "c_model")
     os.makedirs(c_model, exist_ok=True)
-    blocks = [_scalar(N), _scalar(maxM), _scalar(maxM0), _scalar(int(efC)), _scalar(max_level), _scalar(init_node),
-              _scalar(N), _scalar(d), _scalar(maxM0), _scalar(rec)] + _vector(mem_start) + _vector(l0.reshape(-1)) + \
-             [_scalar(N), _scalar(max_level), _scalar(maxM), _scalar(node_mem), _scalar(level_mem)] + _vector(l1)
     write_mmap_store(os.path.join(c_model, "index.mmap_store"), blocks)
     with open(os.path.join(c_model, "config.json"), "w", encoding="utf-8") as f:
-        json.dump({"hnsw_t": _HNSW_T[metric], "version": "v2.0",
-                   "train_params": {"num_node": N, "maxM": maxM, "maxM0": maxM0, "efC": int(efC), "max_level": max_level,
+        json.dump({"hnsw_t": hnsw_t, "version": "v2.0",
+                   "train_params": {"num_node": N, "maxM": maxM, "maxM0": maxM0, "efC": efC, "max_level": max_level,
                                     "init_node": init_node}}, f, indent=4)
     pk = {"efS": 100, "topk": 10, "threads": 1}
     pk.update(pred_kwargs or {})
     with open(os.path.join(folder, "param.json"), "w", encoding="utf-8") as f:
-        json.dump({"model": "HNSW", "data_type": "drm", "metric_type": metric, "num_item": N, "feat_dim": d,
-                   "train_kwargs": {"M": maxM, "efC": int(efC), "builder": "pecos_b200.hnsw_build (batch, exact kNN + heuristic)"},
+        json.dump({"model": "HNSW", "data_type": data_type, "metric_type": metric, "num_item": N, "feat_dim": d,
+                   "train_kwargs": {"M": maxM, "efC": efC, "builder": builder},
                    "pred_kwargs": pk}, f, indent=1)
-    return {"num_node": N, "feat_dim": d, "max_level": max_level, "init_node": init_node,
-            "mean_degree_l0": float(deg0.mean()), "nodes_per_level": [int(t[0].size) for t in level_lists]}
+
+
+# ------------------------------------------------------------------------------------------------ sparse (csr) indices
+_HNSW_T_SPARSE = {
+    "ip": "pecos::ann::HNSW<float, pecos::ann::FeatVecSparseIPSimd<uint32_t, float>>",
+    "l2": "pecos::ann::HNSW<float, pecos::ann::FeatVecSparseL2Simd<uint32_t, float>>",
+}
+
+
+def _is_sparse(X):
+    import scipy.sparse as smat
+
+    return smat.issparse(X)
+
+
+def canonical_csr(X):
+    """The rows the sparse builder indexes and stores: a float32 csr copy with duplicates summed and indices sorted, the steps
+    of the reference's ``HNSW.create_pymat``.  Explicit zeros and empty rows stay as given."""
+    import scipy.sparse as smat
+
+    Xc = smat.csr_matrix(X, dtype=np.float32, copy=True)
+    Xc.sum_duplicates()
+    Xc.sort_indices()
+    return Xc
+
+
+def write_sparse_index(folder, X, level_lists, maxM, maxM0, efC, init_node, metric, pred_kwargs=None,
+                       builder="pecos_b200.hnsw_build (batch, exact sparse kNN + heuristic)"):
+    """Writes a csr index in the reference's format.  ``X``: canonical csr rows (``canonical_csr``); ``level_lists[l]`` =
+    (node ids of level l, neighbour lists [n, maxM0 at level 0 / maxM above] global ids with -1 = empty, degrees).
+
+    Sparse GraphL0 (hnsw.hpp:104-178 with FeatVecSparse): the record of node i starts at byte mem_start_of_node[i] (u64, N + 1
+    entries) and is [deg u32][maxM0 ids u32][len u32][len x f32 values][len x u32 indices]; node_mem_size is 0 and feat_dim
+    the number of columns.  Neighbour slots beyond a node's degree are zero."""
+    N, D = X.shape
+    max_level = len(level_lists) - 1
+    ids0, lists0, deg0 = level_lists[0]
+    lens = np.diff(X.indptr).astype(np.int64)
+    head_w = 1 + maxM0
+    words = head_w + 1 + 2 * lens
+    mem_start = np.zeros(N + 1, dtype="<u8")
+    np.cumsum(words * 4, out=mem_start[1:])
+    w0 = (mem_start[:-1] // 4).astype(np.int64)
+    buf = np.zeros(int(mem_start[-1]) // 4, dtype="<u4")
+    head = np.zeros((N, head_w), dtype="<u4")
+    head[ids0, 0] = deg0
+    head[ids0, 1:] = np.where(lists0 >= 0, lists0, 0).astype("<u4")
+    buf[(w0[:, None] + np.arange(head_w)[None, :]).ravel()] = head.ravel()
+    buf[w0 + head_w] = lens
+    row_of = np.repeat(np.arange(N, dtype=np.int64), lens)
+    vpos = w0[row_of] + head_w + 1 + (np.arange(X.nnz, dtype=np.int64) - X.indptr[row_of].astype(np.int64))
+    buf[vpos] = np.ascontiguousarray(X.data, dtype="<f4").view("<u4")
+    buf[vpos + lens[row_of]] = X.indices.astype("<u4")
+    node_mem, level_mem, l1 = _graph_l1(N, max_level, maxM, level_lists)
+    blocks = [_scalar(N), _scalar(maxM), _scalar(maxM0), _scalar(int(efC)), _scalar(max_level), _scalar(init_node),
+              _scalar(N), _scalar(D), _scalar(maxM0), _scalar(0)] + _vector(mem_start) + _vector(buf.view(np.uint8)) + \
+             [_scalar(N), _scalar(max_level), _scalar(maxM), _scalar(node_mem), _scalar(level_mem)] + _vector(l1)
+    _write_folder(folder, blocks, _HNSW_T_SPARSE[metric], "csr", metric, N, D, maxM, maxM0, int(efC), max_level, init_node,
+                  pred_kwargs, builder)
+
+
+class _PhaseTimer(object):
+    """Device time per build phase from CUDA events on the current stream (read once, after the build)."""
+
+    def __init__(self, torch):
+        self.torch, self.marks = torch, []
+
+    def span(self, name):
+        torch = self.torch
+        timer = self
+
+        class _Span(object):
+            def __enter__(self):
+                self.a = torch.cuda.Event(enable_timing=True)
+                self.a.record()
+
+            def __exit__(self, *exc):
+                b = torch.cuda.Event(enable_timing=True)
+                b.record()
+                timer.marks.append((name, self.a, b))
+
+        return _Span()
+
+    def totals(self):
+        self.torch.cuda.synchronize()
+        out = {}
+        for name, a, b in self.marks:
+            out[name] = out.get(name, 0.0) + a.elapsed_time(b)
+        return out
+
+
+def _build_sparse(X, folder, M, efC, metric, seed, max_level_upper_bound, device, pred_kwargs):
+    """GPU build of a csr index: the dense builder's steps (levels, exact prefix kNN, heuristic, reverse links, sorted lists)
+    with every distance computed by the kernels of csrc/hnsw_build_sparse.cu in the reference's exact bits
+    (FeatVecSparse{IP,L2}Simd::distance), all orders by (distance, id); deterministic.  There is no CPU path."""
+    import time
+
+    import torch
+
+    t_start = time.perf_counter()
+    Xc, dev, dev_index, c = _sparse_setup(torch, X, device)
+    N, D = Xc.shape
+    maxM, maxM0 = int(M), 2 * int(M)
+    metric_id = 0 if metric == "ip" else 1
+    levels, max_level, init_node = _levels(N, maxM, seed, max_level_upper_bound)
+    timer = _PhaseTimer(torch)
+    products = 0
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream().cuda_stream
+        rp, ci, cv = _upload_csr(torch, Xc, dev)
+        lvl = torch.from_numpy(levels).to(dev)
+
+        def select(cand, cand_d, cap):
+            cand = cand.contiguous()
+            cand_d = cand_d.contiguous()
+            keep = torch.empty(cand.shape, dtype=torch.uint8, device=dev)
+            rc = c.pb200_hnsw_build_sparse_select(dev_index, stream, cand.shape[0], cand.shape[1], int(cap), metric_id, rp.data_ptr(),
+                                                  ci.data_ptr(), cv.data_ptr(), cand.data_ptr(), cand_d.data_ptr(), keep.data_ptr())
+            if rc != 0:
+                raise RuntimeError("pb200_hnsw_build_sparse_select failed")
+            return keep.bool()
+
+        level_lists = []
+        for l in range(0, max_level + 1):
+            ids = torch.nonzero(lvl >= l).squeeze(1)
+            n = ids.numel()
+            cap = maxM0 if l == 0 else maxM
+            k = min(int(efC), n - 1)
+            if n <= 1 or k <= 0:
+                lists = torch.full((n, cap), -1, dtype=torch.long, device=dev)
+                level_lists.append((ids.cpu().numpy(), lists.cpu().numpy(), np.zeros(n, dtype=np.int64)))
+                continue
+            pos, dist, prod = _sparse_level_knn(torch, c, dev, dev_index, stream, rp, ci, cv, ids, D, k, metric_id, timer)
+            products += prod
+            sel_spans = []
+
+            def timed_select(cand, cand_d, cap_, _spans=sel_spans):
+                a = torch.cuda.Event(enable_timing=True)
+                b = torch.cuda.Event(enable_timing=True)
+                a.record()
+                out = select(cand, cand_d, cap_)
+                b.record()
+                _spans.append((a, b))
+                return out
+
+            with timer.span("link"):
+                lists, deg = _link_level(torch, ids, pos, dist, maxM, cap, timed_select)
+            # the first heuristic call is the forward selection; the rest of the link span is the reverse links
+            timer.marks.append(("selection", sel_spans[0][0], sel_spans[0][1]))
+            level_lists.append((ids.cpu().numpy(), lists.cpu().numpy(), deg.cpu().numpy()))
+        phases = timer.totals()
+    t_w = time.perf_counter()
+    write_sparse_index(folder, Xc, level_lists, maxM, maxM0, efC, init_node, metric, pred_kwargs)
+    writer_s = time.perf_counter() - t_w
+    link = phases.pop("link", 0.0)
+    phase_ms = {"posting_lists": phases.get("posting_lists", 0.0), "knn": phases.get("knn", 0.0),
+                "selection": phases.get("selection", 0.0), "reverse_links": link - phases.get("selection", 0.0),
+                "writer_host": 1000.0 * writer_s}
+    deg0 = level_lists[0][2]
+    return {"num_node": N, "feat_dim": D, "nnz": int(Xc.nnz), "max_level": max_level, "init_node": init_node,
+            "mean_degree_l0": float(deg0.mean()) if N else 0.0, "nodes_per_level": [int(t[0].size) for t in level_lists],
+            "knn_products": products, "phase_ms": phase_ms, "build_seconds": time.perf_counter() - t_start}
+
+
+def _sparse_setup(torch, X, device):
+    """-> (canonical rows, torch device, device index, CUDA library).  Raises when no GPU is there: no CPU path."""
+    from .core import get_clib
+
+    dev = torch.device(device if device is not None else "cuda:0")
+    if dev.type != "cuda":
+        raise RuntimeError(f"the sparse HNSW builder runs on the GPU only (device={device!r}); there is no CPU fallback")
+    if not torch.cuda.is_available():
+        raise RuntimeError("the sparse HNSW builder needs a visible CUDA device; there is no CPU fallback")
+    lib = get_clib()
+    lib.require_gpu()
+    Xc = canonical_csr(X)
+    if Xc.shape[0] < 1:
+        raise ValueError("empty input")
+    if Xc.shape[0] >= 2 ** 31:
+        raise ValueError("the sparse builder takes at most 2^31 - 1 rows")
+    return Xc, dev, dev.index if dev.index is not None else torch.cuda.current_device(), lib.clib_float32
+
+
+def _upload_csr(torch, Xc, dev):
+    return (torch.from_numpy(Xc.indptr.astype(np.int64)).to(dev), torch.from_numpy(Xc.indices.astype(np.int32)).to(dev),
+            torch.from_numpy(Xc.data.astype(np.float32)).to(dev))
+
+
+def sparse_prefix_knn(X, k, metric="ip", ids=None, device=None):
+    """The builder's exact prefix kNN on its own: for every row of ``ids`` (ascending row numbers, default all rows), its ``k``
+    nearest among the EARLIER rows of ``ids``.  Returns numpy (positions into ``ids`` [n, k], distances [n, k]), ascending by
+    (distance, id), -1 / inf where fewer than k earlier rows exist."""
+    import torch
+
+    if metric not in _HNSW_T:
+        raise ValueError(f"metric must be 'ip' or 'l2', got {metric!r}")
+    Xc, dev, dev_index, c = _sparse_setup(torch, X, device)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream().cuda_stream
+        rp, ci, cv = _upload_csr(torch, Xc, dev)
+        ids = torch.arange(Xc.shape[0], device=dev) if ids is None else torch.as_tensor(np.asarray(ids, dtype=np.int64), device=dev)
+        pos, dist, _ = _sparse_level_knn(torch, c, dev, dev_index, stream, rp, ci, cv, ids, Xc.shape[1], int(k),
+                                         0 if metric == "ip" else 1, _PhaseTimer(torch))
+        return pos.cpu().numpy(), dist.cpu().numpy()
+
+
+def _sparse_level_knn(torch, c, dev, dev_index, stream, rp, ci, cv, ids, D, k, metric_id, timer):
+    """Exact prefix kNN of the rows `ids` (ascending) of the csr (rp, ci, cv) on the device: positions into `ids` [n, k] and
+    distances, ascending by (distance, id), -1 / inf where a node has fewer than k earlier nodes; and the product count."""
+    n = ids.numel()
+    with timer.span("posting_lists"):
+        # the level's rows as a csr of positions 0..n-1 and its posting lists (csc, rows ascending)
+        lens = rp[ids + 1] - rp[ids]
+        lrp = torch.zeros(n + 1, dtype=torch.long, device=dev)
+        torch.cumsum(lens, 0, out=lrp[1:])
+        nnz = int(lrp[-1])
+        row_of = torch.repeat_interleave(torch.arange(n, device=dev), lens, output_size=nnz)
+        src = rp[ids][row_of] + torch.arange(nnz, device=dev) - lrp[:-1][row_of]
+        lci, lcv = ci[src].contiguous(), cv[src].contiguous()
+        perm = torch.argsort(lci.long() * n + row_of)
+        post = torch.stack([row_of[perm].int(), lcv[perm].view(torch.int32)], 1).contiguous()
+        df = torch.bincount(lci.long(), minlength=D)
+        pptr = torch.zeros(D + 1, dtype=torch.long, device=dev)
+        torch.cumsum(df, 0, out=pptr[1:])
+        self_pos = torch.empty(max(nnz, 1), dtype=torch.long, device=dev)
+        self_pos[perm] = torch.arange(nnz, device=dev)
+        cursor = torch.empty(max(nnz, 1), dtype=torch.long, device=dev)
+        products = int((df * (df - 1) // 2).sum())
+    with timer.span("knn"):
+        keys = torch.empty((n, k), dtype=torch.long, device=dev)
+        rc = c.pb200_hnsw_build_sparse_knn(dev_index, stream, n, k, metric_id, lrp.data_ptr(), lci.data_ptr(), lcv.data_ptr(),
+                                           pptr.data_ptr(), post.data_ptr(), self_pos.data_ptr(), cursor.data_ptr(), keys.data_ptr())
+        if rc != 0:
+            raise RuntimeError("pb200_hnsw_build_sparse_knn failed")
+    pos, dist = _decode_keys(torch, keys)
+    return pos, dist, products
+
+
+def _decode_keys(torch, keys):
+    """kNN keys (sign-flipped (orderable(distance) << 32 | position), INT64_MAX = empty) -> positions (-1) and distances (inf)."""
+    empty = keys == torch.iinfo(torch.int64).max
+    u = keys ^ torch.iinfo(torch.int64).min
+    pos = u & 0xFFFFFFFF
+    hi = (u >> 32) & 0xFFFFFFFF
+    bits = torch.where(hi >= 0x80000000, hi - 0x80000000, 0xFFFFFFFF - hi)
+    bits = torch.where(bits >= 0x80000000, bits - (1 << 32), bits).to(torch.int32)
+    dist = bits.view(torch.float32)
+    pos = torch.where(empty, torch.full_like(pos, -1), pos)
+    dist = torch.where(empty, torch.full_like(dist, float("inf")), dist)
+    return pos, dist
